@@ -11,7 +11,7 @@ C3, C5) times one render per frame instead, as round 1 did; the C2 single-render
 `single_render`.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4] [--pattern auto|five|single] [--frames F]
-                  [--lanes S] [--impl b200|reference]
+                  [--lanes S] [--impl b200|reference] [--dump-outputs DIR]
 
 Legs (one JSON line, rank 0):
   value        device-resident: inputs in HBM, C ABI driven through the plan objects, the step captured in a CUDA graph
@@ -27,8 +27,9 @@ Legs (one JSON line, rank 0):
   cpu_baseline the CPU oracle (oracle/, kind "port") on the host cores, bounded sample of the same pattern (N = 1 only)
 `--impl reference` times that CPU oracle on the same pattern through the same GaussianRenderer call (reference arm).
 
-Timing: W >= 3 warm-up steps; L2 flushed (256 MiB memset) before every timed step, outside the per-step CUDA event pairs;
-per-rank time = sum of per-step event durations; max over ranks.  Clocks: NVML polled by a thread during the timed region.
+Timing: W >= 3 warm-up steps, then K timed steps in every GPU leg; L2 flushed (256 MiB memset) before every timed
+step, outside the per-step CUDA event pairs; per-rank time = sum of per-step event durations; max over ranks.  Clocks:
+NVML polled by a thread during the timed region.
 """
 from __future__ import annotations
 
@@ -46,6 +47,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 
 from exavatar_release_b200.camera import look_at_cam_param  # noqa: E402
 from exavatar_release_b200.synthetic import WORKLOADS, make_assets, make_grad_image, make_population_assets  # noqa: E402
@@ -82,6 +84,9 @@ def parse():
                     help="single pattern e2e: Gaussian set host->device once per step or once per frame")
     ap.add_argument("--trace-e2e", default=None, help="write a chrome trace (CUPTI via torch.profiler) of one e2e step here")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU budget of the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the timed step computed in its last step as DIR/<name>.npy (float32); the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output")
     return ap.parse_args()
 
 
@@ -414,6 +419,25 @@ def consumed_units(stt):
     return stt["consumed_fwd"] / stt.get("consumed_fwd_div", 4.0), stt["consumed_bwd"] / stt.get("consumed_bwd_div", 4.0)
 
 
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes `arrays` (device tensors) as out_dir/<name>.npy in float32.  When they hold more than DUMP_BYTES, every
+    array keeps the same share of its elements: a sorted sample of its flattened elements drawn with a fixed seed, so
+    every run with the same arguments writes the same positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    keep = min(1.0, DUMP_BYTES / (4 * sum(v.numel() for v in arrays.values())))
+    for name, v in arrays.items():
+        a = v.detach().float().cpu()
+        if keep < 1.0:
+            a = a.reshape(-1)
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[: int(a.numel() * keep)]
+            a = a[idx.sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # pattern "five": ExAvatar's training frame
 # ---------------------------------------------------------------------------------------------------------------
@@ -543,6 +567,15 @@ def bench_five(env, args, wl, wl_key):
         step()
     clocks = ClockSampler(env.local) if rank == 0 else None
     ms_total, wall, launches_eager = env.timed(step, K)
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        # what the step hands its caller: the summed gradients of the three parameter sets, the densification
+        # statistics (both after the lane fold) and the five renders of the step's last frame
+        outputs = {f"grad_{s}_{k}": v for s in ("scene", "human", "human_refined") for k, v in engine.grads(s).items()}
+        outputs.update({f"densify_{k}": v for k, v in stats.items()})
+        for r in FIVE:
+            outputs.update(zip((f"{r}_color", f"{r}_alpha", f"{r}_radii"), engines[(F - 1) % S].render_outputs(r)))
+        outputs = {k: v.clone() for k, v in outputs.items()}
     if clocks is not None and len(clocks.samples) < 20:
         t_end = time.perf_counter() + 0.5
         while time.perf_counter() < t_end and len(clocks.samples) < 40:
@@ -644,7 +677,7 @@ def bench_five(env, args, wl, wl_key):
 
         for _ in range(3):
             sstep()
-        ks = max(3, min(K, 20))
+        ks = K
         ms_s, _, _ = env.timed(sstep, ks)
         strong = {"value": G * ks / (ms_s * 1e-3), "unit": UNIT, "global_batch": G, "frames_per_rank": len(mine),
                   "ms_per_step": ms_s / ks, "steps": ks,
@@ -663,7 +696,7 @@ def bench_five(env, args, wl, wl_key):
              "streams": engine.describe() + f"; {S} training frame(s) in flight"}
     return {"value": fps, "ms_per_step": ms_total / K, "clocks": clk, "launches": int(launches), "roofline": roofline,
             "e2e": e2e, "e2e_eager": e2e_eager, "e2e_merged": e2e_merged, "strong_scaling": strong, "collective": coll,
-            "wall": wall, "config": extra, "warmup": Wm}
+            "wall": wall, "config": extra, "warmup": Wm, "outputs": outputs}
 
 
 def e2e_five(env, args, wl, wl_key, cams, st_w, st_r, scene_a, human_a, refined_a, cap, caps_merged, collectives):
@@ -818,7 +851,7 @@ def e2e_five(env, args, wl, wl_key, cams, st_w, st_r, scene_a, human_a, refined_
 
     for _ in range(3):
         step()
-    ke = max(3, min(K, 20))
+    ke = K
     ms_e, _, _ = env.timed(step, ke)
     if args.trace_e2e and env.rank == 0:
         from torch.profiler import ProfilerActivity, profile
@@ -901,7 +934,7 @@ def e2e_five(env, args, wl, wl_key, cams, st_w, st_r, scene_a, human_a, refined_
 
         for _ in range(2):
             eager_step()
-        kk = max(2, min(K, 5))
+        kk = K
         t0 = time.perf_counter()
         ms_g, _, _ = env.timed(eager_step, kk)
         eager = {"value": world * F * kk / (ms_g * 1e-3), "unit": UNIT, "steps": kk,
@@ -920,7 +953,7 @@ def bench_single(env, args, wl, wl_key, brief=False):
     from exavatar_release_b200.renderer import GaussianRenderer, render_settings
     dev, lib, world, rank = env.dev, env.lib, env.world, env.rank
     dist = env.dist
-    F, K, Wm = args.frames, (min(args.steps, 10) if brief else args.steps), max(args.warmup, 3)
+    F, K, Wm = args.frames, args.steps, max(args.warmup, 3)
     P, H, Wd = wl.n_avatar + wl.n_scene, wl.height, wl.width
     N = H * Wd
     use_sh = wl.sh_degree > 0
@@ -975,6 +1008,13 @@ def bench_single(env, args, wl, wl_key, brief=False):
         step()
     clocks = ClockSampler(env.local) if (rank == 0 and not brief) else None
     ms_total, wall, launches_eager = env.timed(step, K)
+    outputs = None
+    if args.dump_outputs and rank == 0 and not brief:
+        last = lanes.plans[(F - 1) % S]  # frame f runs on lane f mod S
+        outputs = {"color": last.color, "depth": last.depth, "alpha": last.alpha, "radii": last.radii}
+        if wl.backward:  # the gradients summed over the step's frames
+            outputs.update({f"grad_{k}": v for k, v in lanes.views.items()})
+        outputs = {k: v.clone() for k, v in outputs.items()}
     if clocks is not None and len(clocks.samples) < 20:
         t_end = time.perf_counter() + 0.5
         while time.perf_counter() < t_end and len(clocks.samples) < 40:
@@ -1204,7 +1244,7 @@ def bench_single(env, args, wl, wl_key, brief=False):
 
         for _ in range(3):
             e2e_step()
-        ke = max(3, min(K, 20))
+        ke = K
         ms_e, _, _ = env.timed(e2e_step, ke)
         if args.trace_e2e and rank == 0:  # after the timed region: one more step under the profiler
             from torch.profiler import ProfilerActivity, profile
@@ -1239,7 +1279,7 @@ def bench_single(env, args, wl, wl_key, brief=False):
 
             for _ in range(2):
                 eager_step()
-            kk = max(2, min(K, 5))
+            kk = K
             ms_g, _, _ = env.timed(eager_step, kk)
             eager_call[0] = False
             e2e_eager = {"value": world * F * kk / (ms_g * 1e-3), "unit": UNIT, "steps": kk,
@@ -1250,7 +1290,7 @@ def bench_single(env, args, wl, wl_key, brief=False):
 
     return {"value": fps, "ms_per_step": ms_total / K, "clocks": clk, "launches": int(launches), "roofline": roofline,
             "e2e": e2e, "e2e_eager": e2e_eager, "e2e_merged": None, "strong_scaling": None, "collective": None, "wall": wall,
-            "config": {"cuda_graph": graph is not None, "dup_capacity": cap, "lanes": S}, "warmup": Wm}
+            "config": {"cuda_graph": graph is not None, "dup_capacity": cap, "lanes": S}, "warmup": Wm, "outputs": outputs}
 
 
 def run_b200(args):
@@ -1288,6 +1328,8 @@ def run_b200(args):
                 "collective": res["collective"],
                 "single_render": single, "wall_s_timed_region": res["wall"]}
         print(json.dumps(line), flush=True)
+        if res["outputs"] is not None:
+            dump_outputs(args.dump_outputs, res["outputs"])
     if env.world > 1:
         env.dist.destroy_process_group()
     return 0
@@ -1296,6 +1338,8 @@ def run_b200(args):
 def main():
     args = parse()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs records the B200 arm's step; the reference arm writes none")
         return run_reference(args)
     return run_b200(args)
 
