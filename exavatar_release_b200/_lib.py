@@ -83,6 +83,16 @@ B2R_BWD_ACCUMULATE = 1
 B2R_BWD_SCRATCH_ZEROED = 2
 
 
+def read_status(ctx_buf) -> dict:
+    """The B2RStatus block at the head of a device ctx buffer (a uint8 tensor), copied back to the host (synchronises);
+    for tests, bench accounting and overflow checks.  The composites count staged list entries per CTA; consumed_*_div
+    turn those sums into entries per tile."""
+    s = B2RStatus.from_buffer_copy(ctx_buf[: C.sizeof(B2RStatus)].cpu().numpy().tobytes())
+    out = {name: int(getattr(s, name)) for name, _ in B2RStatus._fields_ if name != "reserved"}
+    out.update(consumed_fwd_div=float(CONSUMED_FWD_DIV), consumed_bwd_div=float(CONSUMED_BWD_DIV))
+    return out
+
+
 # every symbol include/b200raster.h declares: (name, restype, argtypes)
 SYMBOLS = [
     ("b2r_abi_version", C.c_int, []),

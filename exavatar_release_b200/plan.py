@@ -13,7 +13,6 @@ bucket that is all-reduced once per step (SURVEY.md section 8e).
 from __future__ import annotations
 
 import ctypes as C
-import os
 from typing import Dict, Optional
 
 import torch
@@ -22,33 +21,42 @@ from . import _lib as L
 from .rasterizer import _f32c, _make_scene, _ptr
 
 
-class FramePlan:
-    def __init__(self, P: int, width: int, height: int, dup_capacity: int, device, sh_coeffs: int = 0,
-                 segmented: bool = True):
+class _Workspace:
+    """The resident workspace of one projection + binning of P Gaussians with a fixed duplicate capacity: ctx block,
+    duplicate ids, scratch, backward scratch, `n_ckpts` checkpoint buffers and the B2RWorkspace over them."""
+
+    def __init__(self, lib, P: int, width: int, height: int, dup_capacity: int, device, n_ckpts: int = 1):
+        self.capacity = int(dup_capacity)
+        self.ctx_bytes = lib.b2r_ctx_bytes(P, width, height)
+        self.ctx_buf = torch.empty(self.ctx_bytes, dtype=torch.uint8, device=device)
+        self.ids = torch.empty(max(self.capacity, 1), dtype=torch.int32, device=device)
+        self.scratch_bytes = lib.b2r_scratch_bytes(P, width, height, self.capacity)
+        self.scratch = torch.empty(self.scratch_bytes, dtype=torch.uint8, device=device)
+        self.bwd_bytes = lib.b2r_backward_scratch_bytes(P)
+        # zero once: every backward leaves it zero again (B2R_BWD_SCRATCH_ZEROED), so no memset node per render
+        self.bwd_scratch = torch.zeros(self.bwd_bytes, dtype=torch.uint8, device=device)
+        # segment table + blend-state checkpoints of a forward composite (lets the backward replay 512-entry list
+        # segments as independent work items); one buffer per view composited from the same lists
+        self.ckpt_bytes = lib.b2r_checkpoint_bytes(width, height, self.capacity)
+        self.ckpts = [torch.empty(self.ckpt_bytes, dtype=torch.uint8, device=device) for _ in range(n_ckpts)]
+        self.ws = L.B2RWorkspace(self.ctx_buf.data_ptr(), self.ctx_bytes, self.ids.data_ptr(), self.capacity,
+                                 self.scratch.data_ptr(), self.scratch_bytes, None, 0, self.ckpts[0].data_ptr(),
+                                 self.ckpt_bytes)
+
+    def status(self) -> dict:
+        return L.read_status(self.ctx_buf)
+
+
+class FramePlan(_Workspace):
+    def __init__(self, P: int, width: int, height: int, dup_capacity: int, device, sh_coeffs: int = 0):
         self.lib = L.load()
         self.P, self.W, self.H, self.M = int(P), int(width), int(height), int(sh_coeffs)
         self.device = torch.device(device)
-        self.capacity = int(dup_capacity)
         dev = self.device
         f = lambda *s: torch.empty(s, dtype=torch.float32, device=dev)
         self.color, self.depth, self.alpha = f(3, height, width), f(1, height, width), f(1, height, width)
         self.radii = torch.empty(P, dtype=torch.int32, device=dev)
-        self.ctx_bytes = self.lib.b2r_ctx_bytes(P, width, height)
-        self.ctx_buf = torch.empty(self.ctx_bytes, dtype=torch.uint8, device=dev)
-        self.ids = torch.empty(max(self.capacity, 1), dtype=torch.int32, device=dev)
-        self.scratch_bytes = self.lib.b2r_scratch_bytes(P, width, height, self.capacity)
-        self.scratch = torch.empty(self.scratch_bytes, dtype=torch.uint8, device=dev)
-        self.bwd_bytes = self.lib.b2r_backward_scratch_bytes(P)
-        # zero once: every backward leaves it zero again (B2R_BWD_SCRATCH_ZEROED), so no memset node per render
-        self.bwd_scratch = torch.zeros(self.bwd_bytes, dtype=torch.uint8, device=dev)
-        # segment table + blend-state checkpoints of the forward composite (lets the backward replay 512-entry list
-        # segments as independent work items); `segmented=False` reproduces the round-1 whole-list backward
-        segmented = segmented and os.environ.get("B2R_SEGMENTED", "1") != "0"  # A/B switch for measurements
-        self.ckpt_bytes = self.lib.b2r_checkpoint_bytes(width, height, self.capacity) if segmented else 0
-        self.ckpt = torch.empty(max(self.ckpt_bytes, 1), dtype=torch.uint8, device=dev) if segmented else None
-        self.ws = L.B2RWorkspace(self.ctx_buf.data_ptr(), self.ctx_bytes, self.ids.data_ptr(), self.capacity,
-                                 self.scratch.data_ptr(), self.scratch_bytes, None, 0,
-                                 self.ckpt.data_ptr() if segmented else None, self.ckpt_bytes)
+        super().__init__(self.lib, self.P, self.W, self.H, dup_capacity, dev)
         self.out = L.B2RForwardOutputs(self.color.data_ptr(), self.depth.data_ptr(), self.alpha.data_ptr(),
                                        self.radii.data_ptr())
         self._scenes = {}
@@ -93,15 +101,6 @@ class FramePlan:
             st = torch.cuda.current_stream(self.device).cuda_stream
             L.check(self.lib.b2r_backward(C.byref(sc), C.byref(self.ws), C.byref(a), self.bwd_scratch.data_ptr(),
                                           self.bwd_bytes, st), "b2r_backward")
-
-    def status(self) -> dict:
-        raw = self.ctx_buf[: C.sizeof(L.B2RStatus)].cpu().numpy().tobytes()
-        s = L.B2RStatus.from_buffer_copy(raw)
-        return {"num_dups": int(s.num_dups), "dup_capacity": int(s.dup_capacity), "overflow": int(s.overflow),
-                "num_visible": int(s.num_visible), "consumed_fwd": int(s.consumed_fwd),
-                "consumed_bwd": int(s.consumed_bwd),
-                # the composites count staged list entries per CTA; these divisors turn the sums into entries per TILE
-                "consumed_fwd_div": float(L.CONSUMED_FWD_DIV), "consumed_bwd_div": float(L.CONSUMED_BWD_DIV)}
 
 
 def grad_bucket(P: int, device, sh_coeffs: int = 0):
@@ -308,24 +307,14 @@ class FiveRenderPlan:
         return any(p.status()["overflow"] for p in self.plans.values())
 
 
-class _Pass:
+class _Pass(_Workspace):
     """One projection + binning of cat(scene, X) and the views composited from it (MergedFivePlan)."""
 
-    def __init__(self, lib, P, W, H, cap, n_views, device):
+    def __init__(self, lib, P, W, H, dup_capacity, n_views, device):
         dev = device
-        self.P, self.cap = P, int(cap)
-        self.ctx_bytes = lib.b2r_ctx_bytes(P, W, H)
-        self.ctx_buf = torch.empty(self.ctx_bytes, dtype=torch.uint8, device=dev)
-        self.ids = torch.empty(max(self.cap, 1), dtype=torch.int32, device=dev)
-        self.scratch_bytes = lib.b2r_scratch_bytes(P, W, H, self.cap)
-        self.scratch = torch.empty(self.scratch_bytes, dtype=torch.uint8, device=dev)
-        self.bwd_bytes = lib.b2r_backward_scratch_bytes(P)
-        self.bwd_scratch = torch.zeros(self.bwd_bytes, dtype=torch.uint8, device=dev)  # stays zero across renders
-        self.ck_bytes = lib.b2r_checkpoint_bytes(W, H, self.cap)
-        self.ck = [torch.empty(self.ck_bytes, dtype=torch.uint8, device=dev) for _ in range(n_views)]
+        super().__init__(lib, P, W, H, dup_capacity, dev, n_views)
+        self.P = P
         self.radii = torch.empty(P, dtype=torch.int32, device=dev)
-        self.ws = L.B2RWorkspace(self.ctx_buf.data_ptr(), self.ctx_bytes, self.ids.data_ptr(), self.cap,
-                                 self.scratch.data_ptr(), self.scratch_bytes, None, 0, self.ck[0].data_ptr(), self.ck_bytes)
         f = lambda *s: torch.empty(s, dtype=torch.float32, device=dev)
         self.img = [(f(3, H, W), f(1, H, W), f(1, H, W)) for _ in range(n_views)]
         self.state = [(f(H * W), torch.empty(H * W, dtype=torch.int32, device=dev)) for _ in range(n_views)]
@@ -333,12 +322,6 @@ class _Pass:
         self.cat = {k: f(P, w) for k, w in widths.items()}
         self.streams = [torch.cuda.Stream(dev) for _ in range(n_views)]
         self.primed = False
-
-    def status(self) -> dict:
-        raw = self.ctx_buf[: C.sizeof(L.B2RStatus)].cpu().numpy().tobytes()
-        s = L.B2RStatus.from_buffer_copy(raw)
-        return {"num_dups": int(s.num_dups), "overflow": int(s.overflow), "consumed_fwd": int(s.consumed_fwd),
-                "consumed_bwd": int(s.consumed_bwd)}
 
 
 class MergedFivePlan:
@@ -358,7 +341,6 @@ class MergedFivePlan:
     the projection / scatter / sort work.  Interface of FiveRenderPlan."""
     PER = FiveRenderPlan.PER
     VIEWS = {"A": ("scene", "human", "scene_human"), "B": ("human_refined", "scene_human_refined")}
-    SKIP = os.environ.get("B2R_SKIP_TILES", "1") != "0"  # A/B switch of the skipped human-free tiles
 
     def __init__(self, P_scene: int, P_human: int, width: int, height: int, caps: Optional[Dict[str, int]], device):
         self.lib = L.load()
@@ -391,38 +373,104 @@ class MergedFivePlan:
                 buf[: self.Ps].copy_(scene_assets[k].reshape(self.Ps, -1))
 
     def _scene_desc(self, key, ps, settings):
-        """B2RScene of a pass for one camera; cached under `key` (the settings' tensors are then kept alive), or built
-        afresh when key[0] is None (a caller with a new camera every frame)."""
+        """B2RScene of a pass for one camera; cached under `key` (the settings' tensors are then kept alive), or, when
+        key[0] is None (a caller with a new camera every frame), kept only until the pass is used again."""
+        if key[0] is not None and key in self._scenes:
+            return self._scenes[key][0]
+        entry = _make_scene(settings, ps.cat["mean_3d"], None, ps.cat["rgb"], ps.cat["opacity"], ps.cat["scale"],
+                            ps.cat["rotation"], None, 0)
         if key[0] is None:
-            sc, keep = _make_scene(settings, ps.cat["mean_3d"], None, ps.cat["rgb"], ps.cat["opacity"], ps.cat["scale"],
-                                   ps.cat["rotation"], None, 0)
-            ps.last_scene = (sc, keep)  # alive until the pass is used again
-            return sc
-        if key not in self._scenes:
-            sc, keep = _make_scene(settings, ps.cat["mean_3d"], None, ps.cat["rgb"], ps.cat["opacity"], ps.cat["scale"],
-                                   ps.cat["rotation"], None, 0)
-            self._scenes[key] = (sc, keep)
-        return self._scenes[key][0]
+            ps.last_scene = entry
+        else:
+            self._scenes[key] = entry
+        return entry[0]
 
-    def _view(self, ps, v, name, bg):
+    def _human_bg(self, settings_human_bg) -> torch.Tensor:
+        bg_h = _f32c(settings_human_bg.bg.to(self.device), "bg")
+        self._keep.append(bg_h)  # the human-only views point at it until their composites have run
+        del self._keep[:-64]
+        return bg_h
+
+    # ---- the stages of a frame; each enqueues on the stream that is current when it is called ----
+    def _project_bin(self, pk, key, settings, src):
+        """Projection + binning of pass `pk`; returns its B2RScene.  `src`: the human (A) or refined (B) assets, copied
+        into the rows after the scene prefix; None when the caller already wrote them into `passes[pk].cat`."""
+        ps = self.passes[pk]
+        if src is not None:
+            for k, buf in ps.cat.items():
+                buf[self.Ps:].copy_(src[k].reshape(self.Ph, -1))
+        sc = self._scene_desc((key, pk), ps, settings)
+        sc.flags = L.B2R_FLAG_CTX_CLEAN if ps.primed else 0  # every pass leaves its ctx counters zero
+        ps.primed = True
+        st = torch.cuda.current_stream(self.device).cuda_stream
+        L.check(self.lib.b2r_forward_project(C.byref(sc), C.byref(ps.ws), ps.radii.data_ptr(), st), "b2r_forward_project")
+        L.check(self.lib.b2r_forward_bin(C.byref(sc), C.byref(ps.ws), st), "b2r_forward_bin")
+        return sc
+
+    def _forward_composite(self, pk, v, sc, bg_h, scene_done):
+        """Forward composite of view `v` of pass `pk`; returns its B2RView, which the view's backward needs.  Every view
+        but the scene-only one skips the tiles no human Gaussian reaches: a combined view equals the scene-only view
+        there and carries no gradient; a human-only view shows the bare background there.  Both are pre-filled here.
+        `scene_done` is recorded after the scene-only view and waited on before a combined view's pre-fill."""
+        ps, name = self.passes[pk], self.VIEWS[pk][v]
+        st = torch.cuda.current_stream(self.device)
+        color, depth, alpha = ps.img[v]
+        human_only = name in ("human", "human_refined")
+        if human_only:  # bare background, no depth / alpha
+            color.copy_(bg_h.view(3, 1, 1).expand_as(color))
+            depth.zero_()
+            alpha.zero_()
+        elif name != "scene":  # the scene-only render; the composite overwrites the tiles a human Gaussian reaches
+            st.wait_event(scene_done)
+            for dst, src in zip(ps.img[v], self.passes["A"].img[0]):
+                dst.copy_(src)
         lo, hi = self.ranges[name]
         fT, nc = ps.state[v]
-        # Tiles no human Gaussian reaches: a combined view equals the scene-only view there and carries no gradient; a
-        # human-only view shows the bare background there.  Both are pre-filled by the caller and skipped by the kernels.
-        skip = self.Ps if (self.SKIP and name != "scene") else 0
-        return L.B2RView(lo, hi, _ptr(bg), fT.data_ptr(), nc.data_ptr(), ps.ck[v].data_ptr(), ps.ck_bytes, skip, 0)
+        view = L.B2RView(lo, hi, _ptr(bg_h if human_only else None), fT.data_ptr(), nc.data_ptr(),
+                         ps.ckpts[v].data_ptr(), ps.ckpt_bytes, 0 if name == "scene" else self.Ps, 0)
+        out = L.B2RForwardOutputs(color.data_ptr(), depth.data_ptr(), alpha.data_ptr(), ps.radii.data_ptr())
+        L.check(self.lib.b2r_forward_composite(C.byref(sc), C.byref(ps.ws), C.byref(view), C.byref(out), st.cuda_stream),
+                "b2r_forward_composite")
+        if name == "scene":
+            scene_done.record(st)
+        return view
+
+    def _backward_composite(self, pk, v, sc, view, g_color, g_depth=None, g_alpha=None):
+        """Backward composite of view `v` of pass `pk`: adds the view's screen-space gradients into the pass's scratch."""
+        ps = self.passes[pk]
+        a = L.B2RBackwardArgs(_ptr(g_color), _ptr(g_depth), _ptr(g_alpha))
+        a.flags = L.B2R_BWD_SCRATCH_ZEROED
+        a.first_row = self.first_row[self.VIEWS[pk][v]]
+        L.check(self.lib.b2r_backward_composite(C.byref(sc), C.byref(ps.ws), C.byref(view), C.byref(a),
+                                                ps.bwd_scratch.data_ptr(), ps.bwd_bytes,
+                                                torch.cuda.current_stream(self.device).cuda_stream),
+                "b2r_backward_composite")
+
+    def _backward_project(self, pk, sc, g, accumulate, densify):
+        """Backward projection of pass `pk`: writes (accumulate: adds) the gradients of its rows into the `_views_of`
+        dict `g` (pass A: scene rows then human rows; pass B: refined rows).  `densify` is fed by pass A's scene rows."""
+        ps = self.passes[pk]
+        a = L.B2RBackwardArgs(None, None, None, _ptr(g["means3D"]), _ptr(g["means2D"]), None, _ptr(g["colors"]),
+                              _ptr(g["opacities"]), _ptr(g["scales"]), _ptr(g["rotations"]), None)
+        a.flags = (L.B2R_BWD_ACCUMULATE if accumulate else 0) | L.B2R_BWD_SCRATCH_ZEROED
+        a.first_row = 0 if pk == "A" else self.Ps
+        if pk == "A" and densify is not None:
+            a.densify_grad_accum, a.densify_count = _ptr(densify.get("grad_accum")), _ptr(densify.get("count"))
+            a.densify_radius_max = _ptr(densify.get("radius_max"))
+            a.densify_rows = self.Ps
+        L.check(self.lib.b2r_backward_project(C.byref(sc), C.byref(ps.ws), C.byref(a), ps.bwd_scratch.data_ptr(),
+                                              ps.bwd_bytes, torch.cuda.current_stream(self.device).cuda_stream),
+                "b2r_backward_project")
 
     def frame(self, key, settings, settings_human_bg, scene, human, refined, g_colors: Dict[str, torch.Tensor],
               accumulate: bool, densify: Optional[Dict[str, torch.Tensor]] = None, serial: bool = False, probe=None) -> None:
-        """`probe(label)` (serial mode): called after every stage -- bench.py reads the in-library profiler there to get
-        per-view kernel times."""
-        lib = self.lib
+        """Forward + backward of the five renders of one frame.  `serial`: everything on the caller's stream, one stage
+        after the other.  `probe(label)` (serial mode only) is called after every stage with the label "{pass}:bin",
+        "{pass}:{view}:fwd", "{pass}:{view}:bwd" or "{pass}:project_bwd" -- bench.py reads the in-library profiler
+        there to get per-view kernel times."""
         probe = probe if (probe is not None and serial) else (lambda label: None)
         cur = torch.cuda.current_stream(self.device)
-        bg_h = _f32c(settings_human_bg.bg.to(self.device), "bg")
-        self._keep.append(bg_h)
-        del self._keep[:-64]
-        scene_img = self.passes["A"].img[0]  # the scene-only view: what the combined views equal away from the human
+        bg_h = self._human_bg(settings_human_bg)
         scene_done = torch.cuda.Event()
         for pk, names in self.VIEWS.items():
             ps = self.passes[pk]
@@ -430,60 +478,23 @@ class MergedFivePlan:
             if not serial:
                 st.wait_stream(cur)
             with torch.cuda.stream(st):
-                src = human if pk == "A" else refined
-                for k, buf in ps.cat.items():
-                    buf[self.Ps:].copy_(src[k].reshape(self.Ph, -1))
-                sc = self._scene_desc((key, pk), ps, settings)
-                sc.flags = L.B2R_FLAG_CTX_CLEAN if ps.primed else 0  # every pass leaves its ctx counters zero
-                ps.primed = True
-                sp = st.cuda_stream
-                L.check(lib.b2r_forward_project(C.byref(sc), C.byref(ps.ws), ps.radii.data_ptr(), sp), "b2r_forward_project")
-                L.check(lib.b2r_forward_bin(C.byref(sc), C.byref(ps.ws), sp), "b2r_forward_bin")
+                sc = self._project_bin(pk, key, settings, human if pk == "A" else refined)
                 probe(f"{pk}:bin")
-                views = [self._view(ps, v, n, bg_h if n in ("human", "human_refined") else None) for v, n in enumerate(names)]
                 # forward + backward composite of every view; the views of a pass are independent of each other
                 for v, n in enumerate(names):
                     vs = st if serial else ps.streams[v]
                     if not serial:
                         vs.wait_stream(st)
                     with torch.cuda.stream(vs):
-                        color, depth, alpha = ps.img[v]
-                        if views[v].skip_below and n in ("human", "human_refined"):  # bare background, no depth / alpha
-                            color.copy_(bg_h.view(3, 1, 1).expand_as(color))
-                            depth.zero_()
-                            alpha.zero_()
-                        elif views[v].skip_below:  # pre-fill with the scene-only render; the composite overwrites human tiles
-                            vs.wait_event(scene_done)
-                            for dst, src in zip(ps.img[v], scene_img):
-                                dst.copy_(src)
-                        out = L.B2RForwardOutputs(color.data_ptr(), depth.data_ptr(), alpha.data_ptr(), ps.radii.data_ptr())
-                        L.check(lib.b2r_forward_composite(C.byref(sc), C.byref(ps.ws), C.byref(views[v]), C.byref(out),
-                                                          vs.cuda_stream), "b2r_forward_composite")
-                        if n == "scene":
-                            scene_done.record(vs)
+                        view = self._forward_composite(pk, v, sc, bg_h, scene_done)
                         probe(f"{pk}:{n}:fwd")
-                        a = L.B2RBackwardArgs(_ptr(g_colors[n]))
-                        a.flags = L.B2R_BWD_SCRATCH_ZEROED
-                        a.first_row = self.first_row[n]
-                        L.check(lib.b2r_backward_composite(C.byref(sc), C.byref(ps.ws), C.byref(views[v]), C.byref(a),
-                                                           ps.bwd_scratch.data_ptr(), ps.bwd_bytes, vs.cuda_stream),
-                                "b2r_backward_composite")
+                        self._backward_composite(pk, v, sc, view, g_colors[n])
                         probe(f"{pk}:{n}:bwd")
                 if not serial:
-                    for v in range(len(names)):
-                        st.wait_stream(ps.streams[v])
-                # one backward projection per pass
-                g = self.views_A if pk == "A" else self.views_B
-                a = L.B2RBackwardArgs(None, None, None, _ptr(g["means3D"]), _ptr(g["means2D"]), None, _ptr(g["colors"]),
-                                      _ptr(g["opacities"]), _ptr(g["scales"]), _ptr(g["rotations"]), None)
-                a.flags = (L.B2R_BWD_ACCUMULATE if accumulate else 0) | L.B2R_BWD_SCRATCH_ZEROED
-                a.first_row = 0 if pk == "A" else self.Ps
-                if pk == "A" and densify is not None:
-                    a.densify_grad_accum, a.densify_count = _ptr(densify.get("grad_accum")), _ptr(densify.get("count"))
-                    a.densify_radius_max = _ptr(densify.get("radius_max"))
-                    a.densify_rows = self.Ps
-                L.check(lib.b2r_backward_project(C.byref(sc), C.byref(ps.ws), C.byref(a), ps.bwd_scratch.data_ptr(),
-                                                 ps.bwd_bytes, sp), "b2r_backward_project")
+                    for vs in ps.streams:
+                        st.wait_stream(vs)
+                self._backward_project(pk, sc, self.views_A if pk == "A" else self.views_B, accumulate, densify)
+                probe(f"{pk}:project_bwd")
         if not serial:
             for pk in self.passes:
                 cur.wait_stream(self.pass_streams[pk])
@@ -493,51 +504,24 @@ class MergedFivePlan:
         """Forward of the five renders; images in `render_outputs()`, per-pixel state and checkpoints stay in the plan
         until `backward_frame` (so the plan must not start another frame in between).  copy_inputs=False: the caller
         already wrote the human / refined rows into `passes[*].cat` (a captured graph keeps the copies outside)."""
-        lib = self.lib
         cur = torch.cuda.current_stream(self.device)
-        bg_h = _f32c(settings_human_bg.bg.to(self.device), "bg")
-        self._keep.append(bg_h)
-        del self._keep[:-64]
-        scene_img = self.passes["A"].img[0]
+        bg_h = self._human_bg(settings_human_bg)
         scene_done = torch.cuda.Event()
         self._pending = {}
-        for pk, names in self.VIEWS.items():
+        for pk in self.VIEWS:
             ps = self.passes[pk]
             st = self.pass_streams[pk]
             st.wait_stream(cur)
             with torch.cuda.stream(st):
-                if copy_inputs:
-                    src = human if pk == "A" else refined
-                    for k, buf in ps.cat.items():
-                        buf[self.Ps:].copy_(src[k].reshape(self.Ph, -1))
-                sc = self._scene_desc((key, pk), ps, settings)
-                sc.flags = L.B2R_FLAG_CTX_CLEAN if ps.primed else 0
-                ps.primed = True
-                sp = st.cuda_stream
-                L.check(lib.b2r_forward_project(C.byref(sc), C.byref(ps.ws), ps.radii.data_ptr(), sp), "b2r_forward_project")
-                L.check(lib.b2r_forward_bin(C.byref(sc), C.byref(ps.ws), sp), "b2r_forward_bin")
-                views = [self._view(ps, v, n, bg_h if n in ("human", "human_refined") else None) for v, n in enumerate(names)]
-                self._pending[pk] = (sc, views)
-                for v, n in enumerate(names):
-                    vs = ps.streams[v]
+                sc = self._project_bin(pk, key, settings, (human if pk == "A" else refined) if copy_inputs else None)
+                views = []
+                for v, vs in enumerate(ps.streams):
                     vs.wait_stream(st)
                     with torch.cuda.stream(vs):
-                        color, depth, alpha = ps.img[v]
-                        if views[v].skip_below and n in ("human", "human_refined"):
-                            color.copy_(bg_h.view(3, 1, 1).expand_as(color))
-                            depth.zero_()
-                            alpha.zero_()
-                        elif views[v].skip_below:
-                            vs.wait_event(scene_done)
-                            for dst, src_ in zip(ps.img[v], scene_img):
-                                dst.copy_(src_)
-                        out = L.B2RForwardOutputs(color.data_ptr(), depth.data_ptr(), alpha.data_ptr(), ps.radii.data_ptr())
-                        L.check(lib.b2r_forward_composite(C.byref(sc), C.byref(ps.ws), C.byref(views[v]), C.byref(out),
-                                                          vs.cuda_stream), "b2r_forward_composite")
-                        if n == "scene":
-                            scene_done.record(vs)
-                for v in range(len(names)):
-                    st.wait_stream(ps.streams[v])
+                        views.append(self._forward_composite(pk, v, sc, bg_h, scene_done))
+                self._pending[pk] = (sc, views)
+                for vs in ps.streams:
+                    st.wait_stream(vs)
         for pk in self.passes:
             cur.wait_stream(self.pass_streams[pk])
 
@@ -548,7 +532,6 @@ class MergedFivePlan:
         """Backward of the frame `forward_frame` rendered.  g_colors[name] = dL/dimage of a render, or None when the render
         was not used downstream.  grads_A / grads_B: `_views_of`-style dicts with P / P_human rows (pass A: scene rows then
         human rows; pass B: refined rows)."""
-        lib = self.lib
         cur = torch.cuda.current_stream(self.device)
         for pk, names in self.VIEWS.items():
             ps = self.passes[pk]
@@ -565,26 +548,11 @@ class MergedFivePlan:
                     with torch.cuda.stream(vs):
                         if gc is None:
                             gc = torch.zeros(3, self.H, self.W, dtype=torch.float32, device=self.device)
-                        a = L.B2RBackwardArgs(_ptr(gc), _ptr(gd), _ptr(ga))
-                        a.flags = L.B2R_BWD_SCRATCH_ZEROED
-                        a.first_row = self.first_row[n]
-                        L.check(lib.b2r_backward_composite(C.byref(sc), C.byref(ps.ws), C.byref(views[v]), C.byref(a),
-                                                           ps.bwd_scratch.data_ptr(), ps.bwd_bytes, vs.cuda_stream),
-                                "b2r_backward_composite")
+                        self._backward_composite(pk, v, sc, views[v], gc, gd, ga)
                         self._keep.append((gc, gd, ga))
-                for v in range(len(names)):
-                    st.wait_stream(ps.streams[v])
-                g = grads_A if pk == "A" else grads_B
-                a = L.B2RBackwardArgs(None, None, None, _ptr(g["means3D"]), _ptr(g["means2D"]), None, _ptr(g["colors"]),
-                                      _ptr(g["opacities"]), _ptr(g["scales"]), _ptr(g["rotations"]), None)
-                a.flags = (L.B2R_BWD_ACCUMULATE if accumulate else 0) | L.B2R_BWD_SCRATCH_ZEROED
-                a.first_row = 0 if pk == "A" else self.Ps
-                if pk == "A" and densify is not None:
-                    a.densify_grad_accum, a.densify_count = _ptr(densify.get("grad_accum")), _ptr(densify.get("count"))
-                    a.densify_radius_max = _ptr(densify.get("radius_max"))
-                    a.densify_rows = self.Ps
-                L.check(lib.b2r_backward_project(C.byref(sc), C.byref(ps.ws), C.byref(a), ps.bwd_scratch.data_ptr(),
-                                                 ps.bwd_bytes, st.cuda_stream), "b2r_backward_project")
+                for vs in ps.streams:
+                    st.wait_stream(vs)
+                self._backward_project(pk, sc, grads_A if pk == "A" else grads_B, accumulate, densify)
         for pk in self.passes:
             cur.wait_stream(self.pass_streams[pk])
 

@@ -266,10 +266,7 @@ def overflowed() -> bool:
 
 def read_status(cx: _Context) -> dict:
     """Copies the device status block back (synchronises); for tests, bench accounting and debugging."""
-    raw = cx.ctx_buf[: C.sizeof(L.B2RStatus)].cpu().numpy().tobytes()
-    s = L.B2RStatus.from_buffer_copy(raw)
-    return {"num_dups": int(s.num_dups), "dup_capacity": int(s.dup_capacity), "overflow": int(s.overflow),
-            "num_visible": int(s.num_visible), "consumed_fwd": int(s.consumed_fwd), "consumed_bwd": int(s.consumed_bwd)}
+    return L.read_status(cx.ctx_buf)
 
 
 def _backward_impl(cx: _Context, g_color, g_depth, g_alpha, g_posed=None):

@@ -1,7 +1,8 @@
-"""Per-view kernel times of one C4 training frame on MergedFivePlan (serial, in-library CUDA-event profiler).
+"""Per-stage kernel times of one C4 training frame on MergedFivePlan (serial, in-library CUDA-event profiler).
 
   python tools/five_breakdown.py [--workload C4]
-Prints, for each pass, the chain kernels and, for each view, the forward / backward composite duration.
+Runs `MergedFivePlan.frame` in serial mode and prints, after each stage (a pass's projection + binning, the forward /
+backward composite of each view, a pass's backward projection), the kernels it ran and their microseconds.
 """
 import argparse
 import ctypes as C
@@ -44,7 +45,6 @@ def main():
     cnt = (C.c_uint64 * 9)()
     names = [lib.b2r_kernel_name(i).decode() for i in range(9)]
 
-    # replicate MergedFivePlan.frame step by step, reading the profiler after every stage
     def read(label):
         torch.cuda.synchronize()
         lib.b2r_profile_read(ms, cnt, 1)
@@ -53,39 +53,7 @@ def main():
 
     lib.b2r_profile_enable(1)
     lib.b2r_profile_read(ms, cnt, 1)
-    sp = torch.cuda.current_stream(dev).cuda_stream
-    for pk, vnames in plan.VIEWS.items():
-        ps = plan.passes[pk]
-        src = human if pk == "A" else refined
-        for k, buf in ps.cat.items():
-            buf[plan.Ps:].copy_(src[k].reshape(plan.Ph, -1))
-        sc = plan._scene_desc((0, pk), ps, st_w)
-        sc.flags = L.B2R_FLAG_CTX_CLEAN
-        print(f"pass {pk}:")
-        L.check(lib.b2r_forward_project(C.byref(sc), C.byref(ps.ws), ps.radii.data_ptr(), sp), "project")
-        L.check(lib.b2r_forward_bin(C.byref(sc), C.byref(ps.ws), sp), "bin")
-        read("project + bin")
-        bg_h = st_r.bg
-        views = [plan._view(ps, v, n, bg_h if n in ("human", "human_refined") else None) for v, n in enumerate(vnames)]
-        for v, n in enumerate(vnames):
-            color, depth, alpha = ps.img[v]
-            out = L.B2RForwardOutputs(color.data_ptr(), depth.data_ptr(), alpha.data_ptr(), ps.radii.data_ptr())
-            L.check(lib.b2r_forward_composite(C.byref(sc), C.byref(ps.ws), C.byref(views[v]), C.byref(out), sp), "fwd")
-            read(f"view {n}: forward")
-            ab = L.B2RBackwardArgs(g[n].data_ptr())
-            ab.flags = L.B2R_BWD_SCRATCH_ZEROED
-            ab.first_row = plan.first_row[n]
-            L.check(lib.b2r_backward_composite(C.byref(sc), C.byref(ps.ws), C.byref(views[v]), C.byref(ab),
-                                               ps.bwd_scratch.data_ptr(), ps.bwd_bytes, sp), "bwd")
-            read(f"view {n}: backward")
-        gv = plan.views_A if pk == "A" else plan.views_B
-        ab = L.B2RBackwardArgs(None, None, None, gv["means3D"].data_ptr(), gv["means2D"].data_ptr(), None,
-                               gv["colors"].data_ptr(), gv["opacities"].data_ptr(), gv["scales"].data_ptr(),
-                               gv["rotations"].data_ptr(), None)
-        ab.flags = L.B2R_BWD_SCRATCH_ZEROED
-        ab.first_row = 0 if pk == "A" else plan.Ps
-        L.check(lib.b2r_backward_project(C.byref(sc), C.byref(ps.ws), C.byref(ab), ps.bwd_scratch.data_ptr(), ps.bwd_bytes, sp), "pbwd")
-        read("backward projection")
+    plan.frame(0, st_w, st_r, scene, human, refined, g, accumulate=False, serial=True, probe=read)
     lib.b2r_profile_enable(0)
 
 
