@@ -39,6 +39,11 @@ WORKLOADS = {
     "T0": Workload("T0:64x64,300 splats", 64, 64, 150, 150, 0, True),
     "T1": Workload("T1:128x96,4k splats", 96, 128, 2000, 2000, 0, True),
     "T2": Workload("T2:200x136,6k splats,SH3", 136, 200, 3000, 3000, 3, True),
+    # odd image sizes (ExAvatar renders at the size of the input frame): T3's width is not a multiple of 4 (scalar
+    # output stores) and its right / bottom quarter tiles are cut off; T4's right-hand tiles have a half-inside quarter
+    # and a quarter wholly outside, and its bottom tile row a warp whose 8x4 pixel rect lies wholly below the image
+    "T3": Workload("T3:101x77,4k splats", 77, 101, 2000, 2000, 0, True),
+    "T4": Workload("T4:100x68,4k splats", 68, 100, 2000, 2000, 0, True),
 }
 
 

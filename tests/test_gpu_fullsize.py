@@ -5,14 +5,12 @@ VERDICT r01 item 1: C3 (1024x1024, 300 k, SH-3, fwd+bwd), C4 (each of the five r
 against its OWN oracle render, including the detached scene prefix), C5 (1080p, 500 k, fwd), long lists of 600 / 3000 /
 20000 entries in one tile (CTA class, 2-chunk merge, 10-chunk merge).
 """
-import ctypes as C
-
 import numpy as np
 import pytest
 import torch
 
 from parity import compare, contributor_report, last_contributor
-from util import kat_settings, settings_on, workload_settings
+from util import ctx_arrays, kat_settings, settings_on, workload_settings
 from exavatar_release_b200.synthetic import WORKLOADS, make_assets, make_grad_image, make_population_assets
 from oracle import oracle as O
 
@@ -24,22 +22,6 @@ def dev():
     if not torch.cuda.is_available():
         pytest.skip("needs a CUDA device")
     return torch.device("cuda:0")
-
-
-def _ctx_arrays(plan):
-    """(ranges (Tn,2) uint32, ids uint32, n_contrib (H,W) uint32, final_T (H,W) float32) of the plan's last forward."""
-    lib = plan.lib
-    P, W, H = plan.P, plan.W, plan.H
-    tiles = ((W + 15) // 16) * ((H + 15) // 16)
-    buf = plan.ctx_buf.cpu().numpy()
-    base = plan.ctx_buf.data_ptr()
-    off = lambda fn: fn(C.byref(plan.ws), P, W, H) - base
-    take = lambda o, n, dt: np.frombuffer(buf[o:o + n].tobytes(), dt)
-    ranges = take(off(lib.b2r_ctx_ranges), tiles * 8, np.uint32).reshape(tiles, 2)
-    ncon = take(off(lib.b2r_ctx_n_contrib), W * H * 4, np.uint32).reshape(H, W)
-    fT = take(off(lib.b2r_ctx_final_T), W * H * 4, np.float32).reshape(H, W)
-    ids = plan.ids.cpu().numpy().view(np.uint32)
-    return ranges, ids, ncon, fT
 
 
 def _oracle_last(octx):
@@ -75,7 +57,7 @@ def _plan_vs_oracle(dev, case, wl_name, yaw, seed=0, cap=12_000_000, with_da=Fal
     compare(case, "color", plan.color.cpu().numpy(), oc, pm[None], kind="image")
     compare(case, "depth", plan.depth.cpu().numpy(), od, pm[None], kind="image")
     compare(case, "alpha", plan.alpha.cpu().numpy(), oa, pm[None], kind="image")
-    ranges, ids, ncon, fT = _ctx_arrays(plan)
+    ranges, ids, ncon, fT = ctx_arrays(plan.lib, plan, plan.P, plan.W, plan.H)
     contributor_report(case, last_contributor(ids, ranges, ncon, wl.width, wl.height), fT, _oracle_last(octx),
                        octx.final_T(), pm)
     if not wl.backward:
@@ -228,7 +210,7 @@ def test_long_list_sort_is_bit_exact(dev, n):
         plan.forward(sc)
         torch.cuda.synchronize()
         assert plan.status()["overflow"] == 0
-        ranges, ids, ncon, fT = _ctx_arrays(plan)
+        ranges, ids, ncon, fT = ctx_arrays(plan.lib, plan, plan.P, plan.W, plan.H)
         if flags:
             assert plan.status()["num_dups"] == octx.num_dups
             for t in range(ranges.shape[0]):

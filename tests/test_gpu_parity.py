@@ -104,7 +104,7 @@ def _run_pair(dev, wl_name, yaw=12.0, seed=0, with_da=False, bg=(0.2, 0.6, 0.9),
 
 
 @pytest.mark.parametrize("wl,yaw,da", [("T0", 12.0, False), ("T1", 12.0, True), ("T1", -30.0, False), ("T2", 12.0, True),
-                                       ("C1", 12.0, False)])
+                                       ("C1", 12.0, False), ("T3", 12.0, True), ("T4", -20.0, False)])
 def test_forward_backward_parity(dev, wl, yaw, da):
     _run_pair(dev, wl, yaw=yaw, with_da=da)
 
@@ -278,14 +278,14 @@ def test_cov3d_precomp_path(dev):
     _check("d_means3D", m3.grad.cpu().numpy(), og["means3D"], np.broadcast_to(gm[:, None], og["means3D"].shape), max_bad_frac=0.2)
 
 
-@pytest.mark.parametrize("case", ["rgb", "sh", "cov", "depth_alpha_only", "noncontiguous"])
+@pytest.mark.parametrize("case", ["rgb", "sh", "cov", "depth_alpha_only", "noncontiguous", "odd_size"])
 def test_compiled_binding_equals_python_route(dev, monkeypatch, case):
     """The C++ autograd Function (csrc_torch/b2r_torch.cpp) and the Python one (_RasterizeGaussians) are two hosts of the
     same kernels: identical forward outputs bit for bit, gradients equal up to the order of the backward's atomic sums,
-    None exactly where the other route returns None."""
+    None exactly where the other route returns None.  "odd_size": 101x77 (T3), scalar output stores and cut-off tiles."""
     rz = RZ()
     assert rz._compiled_binding(), "the compiled binding (_b2r_torch.so) must be built: python -m exavatar_release_b200.build_ext"
-    wl = "T2" if case == "sh" else "T1"
+    wl = {"sh": "T2", "odd_size": "T3"}.get(case, "T1")
     st = workload_settings(wl, yaw=9.0, device=dev, settings_cls=rz.GaussianRasterizationSettings)
     if case == "sh":
         st = st._replace(sh_degree=3)
@@ -316,7 +316,7 @@ def test_compiled_binding_equals_python_route(dev, monkeypatch, case):
         color, radii, depth, alpha = out
         if case == "depth_alpha_only":
             loss = (depth * gi[:1]).sum() + (alpha * gi[1:2]).sum()
-        elif case == "rgb":
+        elif case in ("rgb", "odd_size"):
             loss = (color * gi).sum() + 0.3 * (depth * gi[:1]).sum()
         else:
             loss = (color * gi).sum()
@@ -619,26 +619,28 @@ def test_unused_outputs_get_no_materialised_gradients(dev):
     assert float(lv1["rgb"].grad.abs().max()) == 0.0
 
 
-@pytest.mark.parametrize("engine", ["merged", "separate"])
-def test_five_render_plan_matches_the_reference_pattern(dev, engine):
+@pytest.mark.parametrize("engine,wl_name", [("merged", "T1"), ("separate", "T1"), ("merged", "T3"), ("separate", "T3")],
+                         ids=["merged", "separate", "T3-merged", "T3-separate"])
+def test_five_render_plan_matches_the_reference_pattern(dev, engine, wl_name):
     """FiveRenderPlan (five concurrent renders, detached scene prefix via `first_row`) and MergedFivePlan (two merged
     projection / binning passes, five views; SURVEY 8f-3) == ExAvatar's pattern written
     with the public autograd API: renderer(scene), renderer(human, bg), renderer(cat(scene.detach(), human)), and the
-    same two for the refined human (avatar/main/model.py:81-162), two frames accumulated."""
+    same two for the refined human (avatar/main/model.py:81-162), two frames accumulated; at 128x96 (T1) and at
+    101x77 (T3: cut-off tiles, scalar stores, views pre-filled and composited over partial tiles)."""
     from exavatar_release_b200 import GaussianRenderer
     from exavatar_release_b200.camera import look_at_cam_param
     from exavatar_release_b200.plan import RENDERS, FiveRenderPlan, MergedFivePlan
     from exavatar_release_b200.renderer import render_settings
     from exavatar_release_b200.synthetic import make_population_assets
     rz = RZ()
-    wl = WORKLOADS["T1"]
+    wl = WORKLOADS[wl_name]
     H, W = wl.height, wl.width
-    scene, human, refined = make_population_assets("T1", seed=0, device=dev)
+    scene, human, refined = make_population_assets(wl_name, seed=0, device=dev)
     Ps, Ph = scene["mean_3d"].shape[0], human["mean_3d"].shape[0]
     bg_w, bg_r = torch.ones(3, device=dev), torch.tensor([0.3, 0.7, 0.2], device=dev)
     yaws = (-8.0, 11.0)
     cams = [look_at_cam_param(y, (H, W), device=dev) for y in yaws]
-    gcol = [{r: make_grad_image("T1", 10 * f + j).to(dev) for j, r in enumerate(RENDERS)} for f in range(len(yaws))]
+    gcol = [{r: make_grad_image(wl_name, 10 * f + j).to(dev) for j, r in enumerate(RENDERS)} for f in range(len(yaws))]
 
     # reference pattern through the public API
     lv = {n: {k: v.clone().requires_grad_() for k, v in a.items()} for n, a in (("scene", scene), ("human", human), ("refined", refined))}
@@ -671,24 +673,25 @@ def test_five_render_plan_matches_the_reference_pattern(dev, engine):
     assert float(lv["scene"]["mean_3d"].grad.abs().sum()) > 0 and float(lv["refined"]["rgb"].grad.abs().sum()) > 0
 
 
-@pytest.mark.parametrize("use_graph", [False, True])
-def test_training_frame_renderer_equals_five_renderer_calls(dev, use_graph):
+@pytest.mark.parametrize("use_graph,wl_name", [(False, "T1"), (True, "T1"), (False, "T3"), (True, "T3")],
+                         ids=["False", "True", "T3-False", "T3-True"])
+def test_training_frame_renderer_equals_five_renderer_calls(dev, use_graph, wl_name):
     """`TrainingFrameRenderer` (one autograd call, two merged passes) against the reference's five `GaussianRenderer`
     calls written with the drop-in rasteriser (avatar/main/model.py:117-162): images, masks, radii, and the gradients
     `loss.backward()` leaves in the three asset dicts and in the scene render's mean_2d; a render left out of the loss
     gets no backward launch (eager) or a zero dL/dimage (use_graph: the frame replays two captured CUDA graphs, three
-    frames so that the third is a pure replay with a new camera)."""
+    frames so that the third is a pure replay with a new camera).  At 128x96 (T1) and at 101x77 (T3)."""
     from exavatar_release_b200 import GaussianRenderer, TrainingFrameRenderer
     from exavatar_release_b200.camera import look_at_cam_param
     from exavatar_release_b200.plan import RENDERS
     from exavatar_release_b200.synthetic import make_population_assets
-    wl = WORKLOADS["T1"]
+    wl = WORKLOADS[wl_name]
     H, W = wl.height, wl.width
-    scene, human, refined = make_population_assets("T1", seed=0, device=dev)
+    scene, human, refined = make_population_assets(wl_name, seed=0, device=dev)
     Ps, Ph = scene["mean_3d"].shape[0], human["mean_3d"].shape[0]
     bg_r = torch.tensor([0.3, 0.7, 0.2], device=dev)
-    gcol = {r: make_grad_image("T1", 50 + j).to(dev) for j, r in enumerate(RENDERS)}
-    gmask = make_grad_image("T1", 60).to(dev)[:1]
+    gcol = {r: make_grad_image(wl_name, 50 + j).to(dev) for j, r in enumerate(RENDERS)}
+    gmask = make_grad_image(wl_name, 60).to(dev)[:1]
     used = ("scene", "human", "scene_human", "scene_human_refined")  # human_refined stays out of the loss
     mk = lambda: {n: {k: v.clone().requires_grad_() for k, v in a.items()} for n, a in
                   (("scene", scene), ("human", human), ("refined", refined))}

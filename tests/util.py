@@ -54,6 +54,23 @@ def rel_err(x, y, floor):
     return float(np.max(np.abs(x - y) / np.maximum(np.abs(y), floor)))
 
 
+def ctx_arrays(lib, ws_owner, P, W, H):
+    """(ranges (Tn,2) uint32, ids uint32, n_contrib (H,W) uint32, final_T (H,W) float32) of the last projection +
+    binning (and, for a FramePlan, forward composite) that ran in `ws_owner`'s workspace: a FramePlan or a pass of a
+    MergedFivePlan (whose views keep their per-pixel state outside the ctx, so there only ranges and ids are theirs)."""
+    import ctypes as C
+    tiles = ((W + 15) // 16) * ((H + 15) // 16)
+    buf = ws_owner.ctx_buf.cpu().numpy()
+    base = ws_owner.ctx_buf.data_ptr()
+    off = lambda fn: fn(C.byref(ws_owner.ws), P, W, H) - base
+    take = lambda o, n, dt: np.frombuffer(buf[o:o + n].tobytes(), dt)
+    ranges = take(off(lib.b2r_ctx_ranges), tiles * 8, np.uint32).reshape(tiles, 2)
+    ncon = take(off(lib.b2r_ctx_n_contrib), W * H * 4, np.uint32).reshape(H, W)
+    fT = take(off(lib.b2r_ctx_final_T), W * H * 4, np.float32).reshape(H, W)
+    ids = ws_owner.ids.cpu().numpy().view(np.uint32)
+    return ranges, ids, ncon, fT
+
+
 def settings_on(st, device, settings_cls):
     """The SAME settings (bit for bit) with their tensors on `device`, as another settings class.  Camera matrices built
     on different devices can differ in the last bit (atan / tan / inverse / mm), which flips radius and tile-rect
