@@ -32,7 +32,7 @@ class B2RScene(C.Structure):
         # fused linear-blend skinning (SURVEY section 8f-2); all NULL / 0 = off
         ("skin_xyz", _fp), ("skin_weights", _fp), ("skin_joint_mats", _fp), ("skin_trans", _fp),
         ("skin_cam_Rinv", _fp), ("skin_cam_t", _fp), ("skin_means_out", _fp), ("skin_J", C.c_int32),
-        ("skin_reserved", C.c_int32),
+        ("sh_rows", C.c_int32),  # two colour sources: SH rows [0, sh_rows), colors_precomp for the rest
     ]
 
 

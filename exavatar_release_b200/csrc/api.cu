@@ -12,6 +12,7 @@ int validate_scene(const B2RScene* sc) {
   if (sc->width > 65535 * TILE || sc->height > 32767 * TILE) return B2R_E_INVALID;
   if (!(sc->tanfovx > 0.f) || !(sc->tanfovy > 0.f)) return B2R_E_INVALID;
   if (!sc->bg || !sc->viewmatrix || !sc->projmatrix || !sc->campos) return B2R_E_INVALID;
+  if (sc->sh_rows < 0 || sc->sh_rows > sc->P) return B2R_E_INVALID;  // SH rows of a two-source scene
   if (sc->P > 0) {
     if (!sc->opacities) return B2R_E_INVALID;
     if (sc->skin_xyz) {  // fused skinning replaces means3D
@@ -21,7 +22,13 @@ int validate_scene(const B2RScene* sc) {
     } else if (!sc->means3D) {
       return B2R_E_INVALID;
     }
-    if ((sc->shs != nullptr) == (sc->colors_precomp != nullptr)) return B2R_E_INVALID;  // exactly one colour source
+    if (sc->sh_rows == 0) {
+      if ((sc->shs != nullptr) == (sc->colors_precomp != nullptr)) return B2R_E_INVALID;  // exactly one colour source
+    } else {  // SH rows [0, sh_rows), colours for the rest
+      if (!sc->shs) return B2R_E_INVALID;
+      if (sc->sh_rows < sc->P && !sc->colors_precomp) return B2R_E_INVALID;
+      if (sc->skin_xyz) return B2R_E_INVALID;
+    }
     const bool sr = sc->scales != nullptr && sc->rotations != nullptr;
     if (sr == (sc->cov3D_precomp != nullptr)) return B2R_E_INVALID;                      // exactly one covariance source
     if ((sc->scales != nullptr) != (sc->rotations != nullptr)) return B2R_E_INVALID;
@@ -45,6 +52,16 @@ int validate_ws(const B2RScene* sc, const B2RWorkspace* ws, bool need_scratch) {
   if (ws->dup_capacity > 0 && !ws->dup_ids) return B2R_E_INVALID;
   if (ws->checkpoints && ws->checkpoint_bytes < b2r_checkpoint_bytes(sc->width, sc->height, ws->dup_capacity)) return B2R_E_WORKSPACE;
   return B2R_OK;
+}
+
+// where the backward projection writes the SH gradient.  One colour source: every row needs dL_dshs.  SH rows
+// [0, sh_rows) before colour rows: the detached prefix may not cut the SH rows (first_row is 0 or >= sh_rows), and
+// dL_dshs may only be NULL when no SH row is past first_row.
+bool sh_grad_ok(const B2RScene* sc, const B2RBackwardArgs* a) {
+  if (sc->sh_rows == 0) return !(sc->shs && a->dL_dshs == nullptr && sc->P > 0);
+  const int64_t fr = (int64_t)a->first_row;
+  if (fr > 0 && fr < sc->sh_rows) return false;
+  return a->dL_dshs != nullptr || fr >= sc->sh_rows;
 }
 
 }  // namespace
@@ -174,8 +191,8 @@ int b2r_backward(const B2RScene* scene, const B2RWorkspace* ws, const B2RBackwar
   rc = validate_ws(scene, ws, false);
   if (rc) return rc;
   if (!args || !args->dL_dcolor || !bwd_scratch) return B2R_E_INVALID;
+  if (!sh_grad_ok(scene, args)) return B2R_E_INVALID;
   if (bwd_scratch_bytes < b2r_backward_scratch_bytes(scene->P)) return B2R_E_WORKSPACE;
-  if (scene->shs && args->dL_dshs == nullptr && scene->P > 0) return B2R_E_INVALID;
   if ((int64_t)args->first_row > (int64_t)scene->P) return B2R_E_INVALID;
   if (args->dL_dposed && !scene->skin_xyz) return B2R_E_INVALID;
   const Ctx cx = resolve(ws, scene->P, scene->width, scene->height);
@@ -207,8 +224,8 @@ int b2r_backward_project(const B2RScene* scene, const B2RWorkspace* ws, const B2
   rc = validate_ws(scene, ws, false);
   if (rc) return rc;
   if (!args || !bwd_scratch) return B2R_E_INVALID;
+  if (!sh_grad_ok(scene, args)) return B2R_E_INVALID;
   if (bwd_scratch_bytes < b2r_backward_scratch_bytes(scene->P)) return B2R_E_WORKSPACE;
-  if (scene->shs && args->dL_dshs == nullptr && scene->P > 0) return B2R_E_INVALID;
   if ((int64_t)args->first_row > (int64_t)scene->P) return B2R_E_INVALID;
   if (args->dL_dposed && !scene->skin_xyz) return B2R_E_INVALID;
   const Ctx cx = resolve(ws, scene->P, scene->width, scene->height);

@@ -62,16 +62,19 @@ __global__ void __launch_bounds__(256, PROJ_MIN_BLOCKS) project_kernel(const B2R
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   // SH rows (192 bytes apart for degree 3) are staged through shared memory: each warp copies the contiguous block of
   // its 32 rows with coalesced 128-byte loads; a thread then reads its own row (odd row stride: conflict-free).
+  // Only rows below sh_rows have coefficients (B2RScene.sh_rows); a warp wholly above them stages nothing and its
+  // lanes take their colour from colors_precomp.
   const float* shrow = nullptr;
   if (sc.shs) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int L = sc.sh_coeffs * 3, S = L | 1;
+    const int sh_rows = sc.sh_rows > 0 ? sc.sh_rows : sc.P;
     float* wstage = reinterpret_cast<float*>(s_cnt + (aggregate ? cx.tiles : 0)) + (size_t)warp * 32 * S;
     const int row0 = blockIdx.x * blockDim.x + warp * 32;
-    const int nrows = min(32, sc.P - row0);
+    const int nrows = min(32, sh_rows - row0);
     if (nrows > 0) stage_rows<0>(wstage, const_cast<float*>(sc.shs) + (size_t)row0 * L, L, nrows, 0xffffffffu);
     __syncwarp();
-    shrow = wstage + lane * S;
+    if (i < sh_rows) shrow = wstage + lane * S;
   }
   // fused skinning: the warp's 32 weight rows (J floats each) take the same staged route as the SH rows
   const float* wrow = nullptr;
@@ -150,7 +153,7 @@ __global__ void __launch_bounds__(256, PROJ_MIN_BLOCKS) project_kernel(const B2R
           const float o = __ldg(sc.opacities + i);
           float rgb[3];
           uint32_t bits = 0;
-          if (sc.shs) {
+          if (shrow) {  // the SH clamp bits are set for SH rows only
             sh_to_rgb(sc.sh_degree, shrow, p, cam, rgb, bits);
           } else {
             rgb[0] = __ldg(sc.colors_precomp + 3 * (size_t)i);

@@ -257,7 +257,14 @@ __device__ __forceinline__ void project_bwd_one(const B2RScene& sc, const Ctx& c
   const float dm2z[3] = {dm2[0], dm2[1], 0.f};
   put3(out.dL_dmeans3D, dm);
   put3(out.dL_dmeans2D, dm2z);
-  put3(out.dL_dcolors, dcol);
+  // a scene with both colour sources (sh_rows > 0): the colour gradient of an SH row went to its coefficients above;
+  // its dL_dcolors row is written zero, or left as it is when accumulating
+  float* dcolors = out.dL_dcolors;
+  if (i < sc.sh_rows) {
+    dcol[0] = dcol[1] = dcol[2] = 0.f;
+    if (accumulate) dcolors = nullptr;
+  }
+  put3(dcolors, dcol);
   put3(out.dL_dscales, dscale);
   if (out.dL_dopacities) {
     if (accumulate) out.dL_dopacities[oi] += dop; else out.dL_dopacities[oi] = dop;
@@ -307,11 +314,14 @@ __global__ void __launch_bounds__(256, PBWD_MIN_BLOCKS) project_bwd_kernel(const
   float* wstage = sh_stage + (size_t)warp * 32 * S;
   const int row0 = blockIdx.x * blockDim.x + warp * 32;
   const int nrows = min(32, sc.P - row0);
-  if (use_sh && nrows > 0) {
-    stage_rows<0>(wstage, const_cast<float*>(sc.shs) + (size_t)row0 * L, L, nrows, 0xffffffffu);
+  // rows [0, sh_rows) are coloured from SH (all rows when B2RScene.sh_rows == 0); the others from colors_precomp
+  const int sh_rows = sc.sh_rows > 0 ? sc.sh_rows : sc.P;
+  const int nsh = min(32, sh_rows - row0);
+  if (use_sh && nsh > 0) {
+    stage_rows<0>(wstage, const_cast<float*>(sc.shs) + (size_t)row0 * L, L, nsh, 0xffffffffu);
     __syncwarp();
   }
-  float* shrow = use_sh ? wstage + lane * S : nullptr;
+  float* shrow = use_sh && i < sh_rows ? wstage + lane * S : nullptr;
   const float* wrow = nullptr;
   if (sc.skin_xyz) {  // skinning weight rows, staged like the SH rows (after them in shared memory)
     const int J = sc.skin_J, SJ = J | 1;
@@ -325,12 +335,13 @@ __global__ void __launch_bounds__(256, PBWD_MIN_BLOCKS) project_bwd_kernel(const
     float4* row = reinterpret_cast<float4*>(const_cast<float*>(gacc)) + 3 * (size_t)i;
     row[0] = row[1] = row[2] = make_float4(0.f, 0.f, 0.f, 0.f);
   }
-  if (use_sh && nrows > 0) {
-    const unsigned rows_active = __ballot_sync(0xffffffffu, active);
+  if (use_sh && nsh > 0) {
+    const unsigned rows_active = __ballot_sync(0xffffffffu, active && i < sh_rows);
     __syncwarp();  // every lane's row is complete before the block is written out cooperatively
-    float* dst = out.dL_dshs + ((ptrdiff_t)row0 - first_row) * L;  // rows below first_row are masked off, never touched
-    if (accumulate) stage_rows<2>(wstage, dst, L, nrows, rows_active);
-    else stage_rows<1>(wstage, dst, L, nrows, rows_active);
+    // rows below first_row and from sh_rows on are masked off, never touched
+    float* dst = out.dL_dshs + ((ptrdiff_t)row0 - first_row) * L;
+    if (accumulate) stage_rows<2>(wstage, dst, L, nsh, rows_active);
+    else stage_rows<1>(wstage, dst, L, nsh, rows_active);
   }
 }
 

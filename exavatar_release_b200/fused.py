@@ -30,6 +30,12 @@ drops from ~2.9 ms (hundreds of stream switches, ctypes calls and small copies) 
 so an otherwise EAGER training loop runs the raster part at graph speed.  Kernel arguments passed by value are frozen in
 the graphs, so a change of the intrinsics (tan fov) re-captures; every render's backward runs (a render left out of the
 loss contributes zeros).
+
+`scene_sh_coeffs=M > 0`: the scene asset dict carries `shs` (P_scene, M, 3) + `sh_degree` in place of `rgb` -- what
+`renderer.scene_gaussian_assets(in_kernel_sh=True)` returns -- and the projection kernel colours the scene Gaussians from
+it (SURVEY.md section 8f-4), in both merged passes.  The gradient reaches `shs` (and through it feature_dc /
+feature_rest) and the scene `mean_3d` gets the view-direction term, as with `GaussianRenderer`.  As there, `shs` is used
+iff `rgb` is absent; a scene whose colour source or M does not match the instance raises a ValueError.
 """
 from __future__ import annotations
 
@@ -38,19 +44,43 @@ from typing import Dict, Optional
 import torch
 from torch import nn
 
-from .plan import RENDERS, MergedFivePlan, _views_of
+from .plan import RENDERS, MergedFivePlan
 from .rasterizer import GaussianRasterizationSettings, _f32c
 from .renderer import render_settings
 
 _KEYS = ("mean_3d", "opacity", "scale", "rotation", "rgb")
-_GRAD_OF = {"mean_3d": "means3D", "opacity": "opacities", "scale": "scales", "rotation": "rotations", "rgb": "colors"}
+_SH_KEYS = ("mean_3d", "opacity", "scale", "rotation", "shs")  # a scene coloured in the kernel
+_GRAD_OF = {"mean_3d": "means3D", "opacity": "opacities", "scale": "scales", "rotation": "rotations", "rgb": "colors",
+            "shs": "shs"}
+
+
+def scene_sh_degree(scene_asset, M: int) -> Optional[int]:
+    """The SH degree of a scene asset dict for a frame renderer built with scene_sh_coeffs = M, or None for an rgb scene.
+    `shs` is used iff `rgb` is absent (GaussianRenderer's rule); a colour source or coefficient count the instance was
+    not built for raises a ValueError."""
+    sh_scene = "rgb" not in scene_asset
+    if sh_scene != (M > 0):
+        raise ValueError(f"TrainingFrameRenderer(scene_sh_coeffs={M}): the scene asset dict carries "
+                         f"{'no rgb' if sh_scene else 'rgb'}; this instance needs {'shs + sh_degree' if M else 'rgb'}")
+    if not sh_scene:
+        return None
+    shs = scene_asset.get("shs")
+    if shs is None or "sh_degree" not in scene_asset or shs.dim() != 3 or tuple(shs.shape[1:]) != (M, 3):
+        raise ValueError(f"TrainingFrameRenderer(scene_sh_coeffs={M}): the scene needs shs of shape (P, {M}, 3) and "
+                         f"sh_degree, got shs {None if shs is None else tuple(shs.shape)}")
+    deg = int(scene_asset["sh_degree"])
+    if not 0 <= deg <= 3 or (deg + 1) ** 2 > M:
+        raise ValueError(f"TrainingFrameRenderer(scene_sh_coeffs={M}): sh_degree {deg} is not in [0, 3] or needs more "
+                         f"than {M} coefficients")
+    return deg
 
 
 class _FrameFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, mod, settings, settings_h, scene_m2d, *tensors):
         plan: MergedFivePlan = mod.plan
-        scene, human, refined = (dict(zip(_KEYS, (_f32c(t.detach(), k) for k, t in zip(_KEYS, tensors[i * 5:i * 5 + 5]))))
+        keys = (mod._scene_keys, _KEYS, _KEYS)
+        scene, human, refined = (dict(zip(keys[i], (_f32c(t.detach(), k) for k, t in zip(keys[i], tensors[i * 5:i * 5 + 5]))))
                                  for i in range(3))
         mod._frame_no += 1
         if mod.use_graph:
@@ -83,16 +113,15 @@ class _FrameFn(torch.autograd.Function):
         if mod.use_graph:
             flat_a, flat_b = mod._graph_backward(gc, gd, ga)  # fresh copies of the resident gradient buffers
         else:
-            flat_a = torch.empty(plan.PER * plan.P, dtype=torch.float32, device=dev)
-            flat_b = torch.empty(plan.PER * plan.Ph, dtype=torch.float32, device=dev)
-        _, va = _views_of(flat_a, plan.P)
-        _, vb = _views_of(flat_b, plan.Ph)
+            flat_a = torch.empty(plan.nA, dtype=torch.float32, device=dev)
+            flat_b = torch.empty(plan.nB, dtype=torch.float32, device=dev)
+        va, vb = plan.grad_views(flat_a, flat_b)
         if not mod.use_graph:
             plan.backward_frame(gc, va, vb, g_depths=gd, g_alphas=ga, densify=mod.densify)
         Ps = plan.Ps
         out = [None, None, None, va["means2D"][:Ps].reshape(ctx.m2d_shape)]
-        for part in (lambda v: v[:Ps], lambda v: v[Ps:]):
-            for k in _KEYS:
+        for keys, part in ((mod._scene_keys, lambda v: v[:Ps]), (_KEYS, lambda v: v[Ps:])):
+            for k in keys:
                 out.append(part(va[_GRAD_OF[k]]))
         for k in _KEYS:
             out.append(vb[_GRAD_OF[k]])
@@ -103,10 +132,12 @@ class _FrameFn(torch.autograd.Function):
 
 class TrainingFrameRenderer(nn.Module):
     def __init__(self, P_scene: int, P_human: int, img_shape, device, dup_capacity: Optional[Dict[str, int]] = None,
-                 use_graph: bool = False, graph_depth_alpha: bool = False):
+                 use_graph: bool = False, graph_depth_alpha: bool = False, scene_sh_coeffs: int = 0):
         super().__init__()
         self.img_shape = (int(img_shape[0]), int(img_shape[1]))
-        self.plan = MergedFivePlan(P_scene, P_human, self.img_shape[1], self.img_shape[0], dup_capacity, device)
+        self.plan = MergedFivePlan(P_scene, P_human, self.img_shape[1], self.img_shape[0], dup_capacity, device,
+                                   scene_sh_coeffs=scene_sh_coeffs)
+        self._scene_keys = _SH_KEYS if self.plan.M else _KEYS
         self.densify = None  # optional {'grad_accum','count','radius_max'} (P_scene) tensors updated by the backward
         self._frame_no = 0
         self.use_graph = bool(use_graph)
@@ -119,9 +150,11 @@ class TrainingFrameRenderer(nn.Module):
             # dL/ddepth and dL/dalpha inputs only when asked for: their backward variant is the slower one
             self._gin_d = {r: torch.zeros(1, H, W, dtype=torch.float32, device=dev) for r in RENDERS} if graph_depth_alpha else None
             self._gin_a = {r: torch.zeros(1, H, W, dtype=torch.float32, device=dev) for r in RENDERS} if graph_depth_alpha else None
-            self._flat_a = torch.zeros(plan.PER * plan.P, dtype=torch.float32, device=dev)
-            self._flat_b = torch.zeros(plan.PER * plan.Ph, dtype=torch.float32, device=dev)
-            self._graphs = {}  # (tanfovx, tanfovy) -> (settings, settings_h, forward graph, backward graph)
+            self._flat_a = torch.zeros(plan.nA, dtype=torch.float32, device=dev)
+            self._flat_b = torch.zeros(plan.nB, dtype=torch.float32, device=dev)
+            # (tanfovx, tanfovy, scale modifier, densify buffers, SH degree) -> (settings, settings_h, forward graph,
+            # backward graph); the SH degree is a by-value kernel argument that grows during training
+            self._graphs = {}
             self._cur = None
 
     # ---- use_graph=True ----
@@ -130,7 +163,7 @@ class TrainingFrameRenderer(nn.Module):
         mk = lambda bg: GaussianRasterizationSettings(
             image_height=settings.image_height, image_width=settings.image_width, tanfovx=settings.tanfovx,
             tanfovy=settings.tanfovy, bg=bg, scale_modifier=settings.scale_modifier, viewmatrix=c[0:16].view(4, 4),
-            projmatrix=c[16:32].view(4, 4), sh_degree=0, campos=c[32:35], prefiltered=False, debug=False)
+            projmatrix=c[16:32].view(4, 4), sh_degree=settings.sh_degree, campos=c[32:35], prefiltered=False, debug=False)
         return mk(c[35:38]), mk(c[38:41])
 
     def _load_inputs(self, settings, settings_h, scene, human, refined):
@@ -142,9 +175,12 @@ class TrainingFrameRenderer(nn.Module):
         c[38:41].copy_(settings_h.bg.reshape(3))
         pa, pb = plan.passes["A"], plan.passes["B"]
         for k in _KEYS:
-            pa.cat[k][: plan.Ps].copy_(scene[k].reshape(plan.Ps, -1))
+            if not (plan.M and k == "rgb"):
+                pa.cat[k][: plan.Ps].copy_(scene[k].reshape(plan.Ps, -1))
             pa.cat[k][plan.Ps:].copy_(human[k].reshape(plan.Ph, -1))
             pb.cat[k][plan.Ps:].copy_(refined[k].reshape(plan.Ph, -1))
+        if plan.M:
+            plan.shs.copy_(scene["shs"].reshape(plan.Ps, plan.M, 3))
 
     def _graph_forward(self, settings, settings_h, scene, human, refined):
         plan = self.plan
@@ -152,15 +188,17 @@ class TrainingFrameRenderer(nn.Module):
         dn = self.densify or {}
         key = (float(settings.tanfovx), float(settings.tanfovy), float(settings.scale_modifier),
                tuple(0 if dn.get(k) is None else dn[k].data_ptr() for k in ("grad_accum", "count", "radius_max")))
+        if plan.M:
+            key += (int(settings.sh_degree),)
         if key not in self._graphs:
             st, st_h = self._resident_settings(settings, settings_h)
             pa, pb = plan.passes["A"], plan.passes["B"]
-            _, va = _views_of(self._flat_a, plan.P)
-            _, vb = _views_of(self._flat_b, plan.Ph)
+            va, vb = plan.grad_views(self._flat_a, self._flat_b)
 
             def fwd():
-                for k in _KEYS:  # the scene rows of pass B come from pass A's copy
-                    pb.cat[k][: plan.Ps].copy_(pa.cat[k][: plan.Ps])
+                for k in _KEYS:  # the scene rows of pass B come from pass A's copy (SH: both read plan.shs)
+                    if not (plan.M and k == "rgb"):
+                        pb.cat[k][: plan.Ps].copy_(pa.cat[k][: plan.Ps])
                 plan.forward_frame(("graph", key), st, st_h, None, None, None, copy_inputs=False)
 
             def bwd():
@@ -203,17 +241,22 @@ class TrainingFrameRenderer(nn.Module):
 
     def forward(self, scene_asset, human_asset, human_asset_refined, cam_param, bg_human, bg=None, raster_settings=None,
                 raster_settings_human=None):
-        """Asset dicts as `GaussianRenderer.forward` takes them (mean_3d, opacity, scale, rotation, rgb); `bg_human` is the
+        """Asset dicts as `GaussianRenderer.forward` takes them (mean_3d, opacity, scale, rotation, rgb -- or, for the scene
+        of an instance built with scene_sh_coeffs > 0, shs + sh_degree in place of rgb); `bg_human` is the
         background of the two human-only renders (model.py:72), `bg` of the others (white by default, module.py:592).
         Returns {render name: {img, depthmap, mask, radius, is_vis[, mean_2d]}} for the five renders of plan.RENDERS."""
         dev = scene_asset["mean_3d"].device
+        deg = scene_sh_degree(scene_asset, self.plan.M)  # raises before anything is enqueued
         if bg is None:
             bg = torch.ones(3, dtype=torch.float32, device=dev)
         st = raster_settings or render_settings(self.img_shape, cam_param, bg, GaussianRasterizationSettings)
+        if deg is not None:
+            st = st._replace(sh_degree=deg)
         st_h = raster_settings_human or st._replace(bg=bg_human)
         Ps = scene_asset["mean_3d"].shape[0]
         mean_2d = torch.zeros((Ps, 3), dtype=torch.float32, device=dev, requires_grad=True)  # module.py:626-629
-        flat = [a[k] for a in (scene_asset, human_asset, human_asset_refined) for k in _KEYS]
+        flat = [a[k] for a, keys in ((scene_asset, self._scene_keys), (human_asset, _KEYS), (human_asset_refined, _KEYS))
+                for k in keys]
         res = _FrameFn.apply(self, st, st_h, mean_2d, *flat)
         radii_a, radii_b = res[15], res[16]
         radius = {"scene": radii_a[:Ps], "human": radii_a[Ps:], "scene_human": radii_a, "human_refined": radii_b[Ps:],

@@ -338,24 +338,37 @@ class MergedFivePlan:
     combined view skips the detached scene prefix, `first_row`), and the backward projection runs once per pass: scene
     rows carry the scene render's gradient, human rows the sum of the human-only and the combined render's -- what
     `loss.backward()` leaves in the leaves of model.py:117-125.  Same results as five separate renders (tests/), 2/5 of
-    the projection / scatter / sort work.  Interface of FiveRenderPlan."""
+    the projection / scatter / sort work.  Interface of FiveRenderPlan.
+
+    scene_sh_coeffs = M > 0 (SURVEY.md section 8f-4 inside the merged frame): the scene Gaussians are coloured from their
+    (P_scene, M, 3) SH coefficients in the projection kernel, as SceneGaussian does in PyTorch (module.py:253-272); the
+    human rows keep their rgb.  One resident SH buffer serves both passes (their scene rows are identical; `set_scene`
+    takes `shs`), each pass is described with B2RScene.sh_rows = P_scene and the frame's `settings.sh_degree`.  Pass A's
+    backward projection writes the SH gradient of the scene rows (`grads("scene")["shs"]`, in place of "colors") and
+    adds the view-direction term to their mean gradient; pass B's scene rows are detached and get nothing."""
     PER = FiveRenderPlan.PER
     VIEWS = {"A": ("scene", "human", "scene_human"), "B": ("human_refined", "scene_human_refined")}
 
-    def __init__(self, P_scene: int, P_human: int, width: int, height: int, caps: Optional[Dict[str, int]], device):
+    def __init__(self, P_scene: int, P_human: int, width: int, height: int, caps: Optional[Dict[str, int]], device,
+                 scene_sh_coeffs: int = 0):
         self.lib = L.load()
         self.Ps, self.Ph, self.P = int(P_scene), int(P_human), int(P_scene) + int(P_human)
+        self.M = int(scene_sh_coeffs)
+        if not 0 <= self.M <= 16 or (self.M > 0 and self.Ps == 0):
+            raise ValueError(f"MergedFivePlan: scene_sh_coeffs must be in [0, 16] with a non-empty scene, got {self.M}")
         self.W, self.H = int(width), int(height)
         self.device = torch.device(device)
         caps = caps or {"A": 8_000_000, "B": 8_000_000}
         self.passes = {k: _Pass(self.lib, self.P, self.W, self.H, caps[k], len(v), self.device) for k, v in self.VIEWS.items()}
         self.pass_streams = {k: torch.cuda.Stream(self.device) for k in self.passes}
-        # one flat gradient buffer: [pass A: scene rows | human rows][pass B: refined rows]
-        nA, nB = self.PER * self.P, self.PER * self.Ph
+        # the scene's SH coefficients, read by the projection of both passes
+        self.shs = torch.zeros(self.Ps, self.M, 3, dtype=torch.float32, device=device) if self.M else None
+        # one flat gradient buffer: [pass A: scene rows | human rows (| scene SH)][pass B: refined rows]
+        self.nA, self.nB = self.PER * self.P + 3 * self.M * self.Ps, self.PER * self.Ph
+        nA, nB = self.nA, self.nB
         self.all_flat = torch.zeros(nA + nB + 2 * self.Ps, dtype=torch.float32, device=device)
         self._stats = self.all_flat[nA + nB:]  # per-step densification sums ride in the all-reduced buffer (stats())
-        _, self.views_A = _views_of(self.all_flat[:nA], self.P)
-        _, self.views_B = _views_of(self.all_flat[nA:], self.Ph)
+        self.views_A, self.views_B = self.grad_views(self.all_flat[:nA], self.all_flat[nA:nA + nB])
         Ps, P = self.Ps, self.P
         self.ranges = {"scene": (0, Ps), "human": (Ps, P), "scene_human": (0, P), "human_refined": (Ps, P),
                        "scene_human_refined": (0, P)}
@@ -367,18 +380,35 @@ class MergedFivePlan:
         return ("two merged passes per frame (cat(scene,human): 3 views; cat(scene,refined): 2 views), each one "
                 "projection + binning + sort; composites of a pass on parallel CUDA streams")
 
+    def grad_views(self, flat_a: torch.Tensor, flat_b: torch.Tensor):
+        """`_views_of`-style dicts over flat pass-A / pass-B gradient buffers of `nA` / `nB` floats.  Pass A: scene rows
+        then human rows, and with an SH scene its (P_scene, M, 3) coefficient gradient under "shs"; pass B: refined rows."""
+        _, va = _views_of(flat_a[: self.PER * self.P], self.P)
+        if self.M:
+            va["shs"] = flat_a[self.PER * self.P:].view(self.Ps, self.M, 3)
+        _, vb = _views_of(flat_b, self.Ph)
+        return va, vb
+
     def set_scene(self, scene_assets: Dict[str, torch.Tensor]) -> None:
+        """Copies the scene Gaussians into the prefix of both passes; with scene_sh_coeffs > 0 `scene_assets` carries
+        `shs` (P_scene, M, 3) in place of `rgb`."""
         for ps in self.passes.values():
             for k, buf in ps.cat.items():
+                if self.M and k == "rgb":
+                    continue
                 buf[: self.Ps].copy_(scene_assets[k].reshape(self.Ps, -1))
+        if self.M:
+            self.shs.copy_(scene_assets["shs"].reshape(self.Ps, self.M, 3))
 
     def _scene_desc(self, key, ps, settings):
         """B2RScene of a pass for one camera; cached under `key` (the settings' tensors are then kept alive), or, when
         key[0] is None (a caller with a new camera every frame), kept only until the pass is used again."""
         if key[0] is not None and key in self._scenes:
             return self._scenes[key][0]
-        entry = _make_scene(settings, ps.cat["mean_3d"], None, ps.cat["rgb"], ps.cat["opacity"], ps.cat["scale"],
+        entry = _make_scene(settings, ps.cat["mean_3d"], self.shs, ps.cat["rgb"], ps.cat["opacity"], ps.cat["scale"],
                             ps.cat["rotation"], None, 0)
+        if self.M:
+            entry[0].sh_rows = self.Ps  # scene rows from SH, human rows from rgb
         if key[0] is None:
             ps.last_scene = entry
         else:
@@ -450,7 +480,7 @@ class MergedFivePlan:
         """Backward projection of pass `pk`: writes (accumulate: adds) the gradients of its rows into the `_views_of`
         dict `g` (pass A: scene rows then human rows; pass B: refined rows).  `densify` is fed by pass A's scene rows."""
         ps = self.passes[pk]
-        a = L.B2RBackwardArgs(None, None, None, _ptr(g["means3D"]), _ptr(g["means2D"]), None, _ptr(g["colors"]),
+        a = L.B2RBackwardArgs(None, None, None, _ptr(g["means3D"]), _ptr(g["means2D"]), _ptr(g.get("shs")), _ptr(g["colors"]),
                               _ptr(g["opacities"]), _ptr(g["scales"]), _ptr(g["rotations"]), None)
         a.flags = (L.B2R_BWD_ACCUMULATE if accumulate else 0) | L.B2R_BWD_SCRATCH_ZEROED
         a.first_row = 0 if pk == "A" else self.Ps
@@ -571,9 +601,12 @@ class MergedFivePlan:
 
     def grads(self, which: str) -> Dict[str, torch.Tensor]:
         if which == "scene":
-            return {k: v[: self.Ps] for k, v in self.views_A.items()}
+            g = {k: v[: self.Ps] for k, v in self.views_A.items()}
+            if self.M:
+                del g["colors"]  # the scene rows' colour gradient went to their SH coefficients
+            return g
         if which == "human":
-            return {k: v[self.Ps:] for k, v in self.views_A.items()}
+            return {k: v[self.Ps:] for k, v in self.views_A.items() if k != "shs"}
         return dict(self.views_B)
 
     def flat_bucket(self) -> torch.Tensor:

@@ -130,3 +130,23 @@ def make_population_assets(workload, seed=0, device="cpu", focal_ratio=1.465):
     refined["rgb"] = (human["rgb"] + 0.05 * torch.randn(wl.n_avatar, 3, generator=g)).clamp(0, 1)
     to = lambda d: {k: v.to(device) for k, v in d.items()}
     return to(scene), to(human), to(refined)
+
+
+def make_scene_sh_params(workload, seed=0, device="cpu", focal_ratio=1.465):
+    """The scene population of `make_population_assets(workload, seed)` as SceneGaussian stores it (module.py:103-108):
+    mean, opacity_logit, log_scale, rotation (activated), feature_dc (P,1,3) and feature_rest (P,15,3) -- degree-3
+    SH as `max_sh_degree = 3` trains it (config.py:15-16).  feature_dc is RGB2SH of the population's rgb
+    (transforms.py:169-170); feature_rest is drawn from a generator of its own, so the other generators' outputs do not
+    change.  Feed them to `renderer.scene_gaussian_assets`."""
+    scene, _, _ = make_population_assets(workload, seed=seed, focal_ratio=focal_ratio)
+    n = scene["mean_3d"].shape[0]
+    g = torch.Generator().manual_seed(3000 + seed)
+    p = {
+        "mean": scene["mean_3d"],
+        "opacity_logit": torch.logit(scene["opacity"].clamp(1e-4, 1 - 1e-4)),
+        "log_scale": torch.log(scene["scale"]),
+        "rotation": scene["rotation"],
+        "feature_dc": ((scene["rgb"] - 0.5) / SH_C0)[:, None, :],
+        "feature_rest": 0.2 * torch.randn(n, 15, 3, generator=g),
+    }
+    return {k: v.contiguous().to(device) for k, v in p.items()}

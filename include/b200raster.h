@@ -53,7 +53,7 @@ extern "C" {
 typedef struct B2RScene {
   int32_t P;              /* number of Gaussians */
   int32_t width, height;  /* image_width, image_height */
-  int32_t sh_degree;      /* active SH degree (0..3); ignored when colors_precomp != NULL */
+  int32_t sh_degree;      /* active SH degree (0..3); ignored when shs == NULL */
   int32_t sh_coeffs;      /* M: coefficients per Gaussian in `shs` (0 when shs == NULL) */
   uint32_t flags;         /* B2R_FLAG_* */
   float scale_modifier;
@@ -63,8 +63,8 @@ typedef struct B2RScene {
   const float* projmatrix;    /* (16) full projection (proj*view), [4c+r] */
   const float* campos;        /* (3) */
   const float* means3D;       /* (P,3) */
-  const float* shs;           /* (P,M,3) or NULL */
-  const float* colors_precomp;/* (P,3) or NULL  (exactly one of shs / colors_precomp) */
+  const float* shs;           /* (P,M,3) or NULL; (sh_rows,M,3) when sh_rows > 0 */
+  const float* colors_precomp;/* (P,3) or NULL  (exactly one of shs / colors_precomp, unless sh_rows > 0: see there) */
   const float* opacities;     /* (P) */
   const float* scales;        /* (P,3) or NULL */
   const float* rotations;     /* (P,4) (r,x,y,z), used un-normalised, or NULL */
@@ -84,7 +84,17 @@ typedef struct B2RScene {
   const float* skin_cam_t;      /* (3) camera translation (used with skin_cam_Rinv) */
   float* skin_means_out;        /* (P,3) optional OUTPUT: the posed world positions (other ExAvatar modules read them) */
   int32_t skin_J;               /* joints (55 for SMPL-X); <= 64 */
-  int32_t skin_reserved;
+  /* Two colour sources in one scene (SURVEY section 8f-4 inside the merged frame of 8f-3): ExAvatar colours its scene
+   * Gaussians from SH and its human Gaussians from rgb, and a merged pass renders cat(scene, human).
+   *   sh_rows == 0:        one colour source for every row -- exactly one of shs (P,M,3) / colors_precomp (P,3).
+   *   0 < sh_rows <= P:    rows [0, sh_rows) are coloured from `shs`, which is then (sh_rows,M,3) at `sh_degree`; rows
+   *                        [sh_rows, P) from `colors_precomp`, which stays (P,3) indexed by Gaussian id (its rows below
+   *                        sh_rows are never read).  colors_precomp is required iff sh_rows < P.  Not with skin_xyz.
+   *   Backward (b2r_backward / b2r_backward_project): rows first_row <= i < sh_rows receive their SH gradient in
+   *   dL_dshs row i - first_row and the view-direction term in dL_dmeans3D; their dL_dcolors row is written zero (left
+   *   untouched with B2R_BWD_ACCUMULATE).  Rows >= sh_rows receive dL_dcolors.  first_row must be 0 or >= sh_rows;
+   *   with first_row >= sh_rows no SH row takes part and dL_dshs may be NULL. */
+  int32_t sh_rows;
 } B2RScene;
 
 /* Device-side status block; lives at offset 0 of the ctx buffer (read it back with a 64-byte D2H copy). */
